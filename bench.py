@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — CTR training samples/s of DeepFM on a synthetic Criteo-shaped batch (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch: clear_grad -> DeepFMLayer.forward (fused
@@ -60,7 +60,13 @@ def parse():
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--timeline", default="", help="write a CUPTI timeline of 3 steps (rank 0) "
                    "as <path>.json (chrome trace) and <path>.txt (per-stream summary) and exit")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", default="", metavar="DIR",
+                   help="after the timed steps write what the last one computed (rank 0) as "
+                        "DIR/<name>.npy, so that two builds can be compared output for output")
+    args = p.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        p.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def algorithmic_bytes_fwd(D, F=F_SPARSE, Dn=N_DENSE):
@@ -258,6 +264,9 @@ def run_b200(args, rank, world, local_rank):
 
     prefetch = getattr(model, "prefetch", None)
     finish_prefetch = getattr(model, "finish_prefetch", None)
+    # detached: a reference to pred or loss would keep the step's autograd graph, and with it the
+    # tower's activation planes, alive into the next step
+    last = {} if args.dump_outputs else None
 
     def step_resident(i):
         label, ids, dense = resident[i % len(resident)]
@@ -270,6 +279,8 @@ def run_b200(args, rank, world, local_rank):
         if finish_prefetch is not None:
             finish_prefetch()
         optimizer.step()
+        if last is not None:
+            last["pred"], last["loss"], last["ids"] = pred.detach(), loss.detach(), ids
         return loss
 
     from paddlerec_b200 import runner
@@ -338,6 +349,8 @@ def run_b200(args, rank, world, local_rank):
     parity = parity_bit(args, model, dm, resident, label_f, rank, world, dev) if world > 1 else None
     ms, launches, events, clocks = timed(step_resident, K, W, collect_events=True,
                                          event_filter={"embed_fm_fwd"})
+    if args.dump_outputs and rank == 0:   # before the passes below train the model further
+        dump_outputs(args.dump_outputs, model, last, args, rank, world)
     value = args.batch * world * K / (ms / 1e3)
     k_ms = [s.elapsed_time(e) for (name, s, e) in events if name == "embed_fm_fwd"]
     kernel_ms = sum(k_ms) / max(len(k_ms), 1)
@@ -448,6 +461,39 @@ def timeline(path, step, barrier, rank, warmup):
             lines.append("%10.1f %9.1f           %s" % (e["ts"] - t0, e["dur"], e["name"][:90]))
     open(path + ".txt", "w").write("\n".join(lines) + "\n")
     print("\n".join(lines[:12]), flush=True)
+
+
+DUMP_TABLE_ROWS = 1 << 16
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, model, last, args, rank, world):
+    """The last timed step's prediction and loss and the parameters it left (state_dict names) as
+    float32 `<name>.npy`.  A table of more than DUMP_TABLE_ROWS rows is written at a fixed, seeded
+    sample of rows, half of them drawn from the ids that step looked up (so rows it updated) and
+    half from all ids; `table_rows.npy` (float64) holds their global ids.  At N>1: rank 0's shard."""
+    import numpy as np
+
+    g = torch.Generator().manual_seed(2024)
+    looked = last["ids"].reshape(-1).cpu()
+    gid = torch.unique(torch.cat([
+        looked[torch.randint(0, looked.numel(), (DUMP_TABLE_ROWS // 2,), generator=g)],
+        torch.randint(0, args.vocab, (DUMP_TABLE_ROWS // 2,), generator=g)]))
+    gid = gid[gid % world == rank]
+    out = {"pred": last["pred"].reshape(-1), "loss": last["loss"].reshape(-1)}
+    for name, t in model.state_dict().items():
+        if t.dim() == 2 and t.shape[0] > DUMP_TABLE_ROWS:
+            t = t[(gid // world).to(t.device)]
+            out["table_rows"] = gid
+        out[name] = t
+    out = {k: v.detach().to("cpu", torch.float64 if k == "table_rows" else torch.float32).numpy()
+           for k, v in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def roofline_step(args, per_ms, step_ms, step_ms_with_events, world):

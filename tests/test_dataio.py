@@ -6,8 +6,8 @@ unmodified) — see tests/golden/make_reader_golden.py.  Integer output (ids, la
 be bit-exact; float32 dense values bit-exact against the Python reader, and within the 6
 significant digits parser.cpp prints against its text output.
 """
+import gzip
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -108,9 +108,7 @@ def test_criteo_tsv_matches_golden_from_reference_parser_cpp():
     assert np.array_equal(od, dense)                          # bit-exact vs the restatement
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "criteo_parser")),
-                    reason="oracle/_ref/criteo_parser not built (needs /root/reference)")
-def test_criteo_tsv_matches_reference_binary_live():
+def _random_criteo_tsv():
     rng = np.random.default_rng(5)
     lines = []
     for _ in range(700):
@@ -118,10 +116,14 @@ def test_criteo_tsv_matches_reference_binary_live():
         cols += ["" if rng.random() < 0.3 else str(rng.integers(-3, 70000)) for _ in range(13)]
         cols += ["" if rng.random() < 0.2 else "%x" % rng.integers(0, 1 << 40) for _ in range(26)]
         lines.append("\t".join(cols))
-    tsv = ("\n".join(lines) + "\n").encode()
-    out = subprocess.run([os.path.join(ROOT, "oracle", "_ref", "criteo_parser")], input=tsv,
-                         capture_output=True, check=True).stdout
-    rl, rid, rd = _parser_cpp_output(out)
+    return ("\n".join(lines) + "\n").encode()
+
+
+def test_criteo_tsv_matches_reference_binary_live():
+    """700 seeded lines against what parser.cpp printed for them (tests/golden/make_live_golden.py)."""
+    tsv = _random_criteo_tsv()
+    rl, rid, rd = _parser_cpp_output(gzip.decompress(_read("criteo_tsv_parser_cpp_live.txt.gz")))
+    assert rid.shape == (700, 26)
     for threads in (1, 3):
         label, ids, dense, skipped = dataio.parse_criteo_tsv(tsv, threads=threads)
         assert skipped == 0 and np.array_equal(ids, rid) and np.array_equal(label[:, 0], rl)

@@ -1,13 +1,14 @@
-"""Live cross-check (authoring container only: needs /root/reference): the reference's own
-models/rank/*/net.py, executed unmodified on oracle/paddle_shim.py with FRESH seeds and shapes,
-against oracle/nets.py — forward and every parameter gradient, float64.  Skipped on the GPU box."""
+"""Cross-check with fresh seeds and shapes: what the reference's own models/rank/*/net.py and readers
+computed, executed unmodified on oracle/paddle_shim.py (recorded by tests/golden/make_live_golden.py),
+against oracle/nets.py, oracle/readers.py and the native parsers — forward and every parameter
+gradient, float64."""
 import os
 
+import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference/models/rank"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(autouse=True)
@@ -18,118 +19,84 @@ def _f64():
     torch.set_default_dtype(prev)
 
 
-def _grads(loss, named):
-    gs = torch.autograd.grad(loss, list(named.values()), allow_unused=True, retain_graph=True)
-    return {k: (torch.zeros_like(p) if g is None else g) for (k, p), g in zip(named.items(), gs)}
+def _case(name):
+    """(parameters as float64 leaves, inputs, reference output, reference gradients) of one case."""
+    z = np.load(os.path.join(GOLD, "reference_live_%s.npz" % name))
+    part = {"param": {}, "in": {}, "grad": {}}
+    for k in z.files:
+        if k != "out":
+            group, _, key = k.partition("/")
+            part[group][key] = z[k]
+    named = {k: torch.tensor(v).requires_grad_(True) for k, v in part["param"].items()}
+    inputs = {k: torch.tensor(v) for k, v in part["in"].items()}
+    return named, inputs, z["out"], part["grad"]
 
 
-def _same(ref_out, ora_out, named):
-    assert (ref_out - ora_out).abs().max() < 1e-12
-    g1 = _grads(ref_out.square().sum(), named)
-    g2 = _grads(ora_out.square().sum(), named)
-    for k in g1:
-        assert (g1[k] - g2[k]).abs().max() < 1e-10, k
+def _slots(ids):
+    return [ids[:, i:i + 1] for i in range(ids.shape[1])]
+
+
+def _same(ref_out, ref_grads, ora_out, named):
+    assert np.abs(ref_out - ora_out.detach().numpy()).max() < 1e-12
+    gs = torch.autograd.grad(ora_out.square().sum(), list(named.values()), allow_unused=True)
+    got = {k: (torch.zeros_like(p) if g is None else g) for (k, p), g in zip(named.items(), gs)}
+    assert set(got) == set(ref_grads)
+    for k in ref_grads:
+        assert np.abs(ref_grads[k] - got[k].numpy()).max() < 1e-10, k
 
 
 @pytest.mark.parametrize("seed,D,B", [(1, 5, 3), (2, 12, 9)])
 def test_deepfm_live(seed, D, B):
-    from oracle import nets, paddle_shim
-    ref = paddle_shim.import_reference_net("deepfm")
-    torch.manual_seed(seed)
-    V, fc = 61, [7, 5, 3]
-    layer = ref.DeepFMLayer(V, D, 13, 26, fc)
-    ids = [torch.randint(0, V, (B, 1)) for _ in range(26)]
-    dense = torch.rand(B, 13)
-    named = dict(layer.named_parameters())
-    _same(layer(ids, dense), nets.deepfm_forward(named, ids, dense, len(fc)), named)
+    from oracle import nets
+    named, i, out, grads = _case("deepfm_%d" % seed)
+    assert i["ids"].shape == (B, 26) and named["fm.embedding.weight"].shape[1] == D
+    _same(out, grads, nets.deepfm_forward(named, _slots(i["ids"]), i["dense"], 3), named)
 
 
 @pytest.mark.parametrize("mix,stacked", [(False, False), (True, True)])
 def test_dcn_v2_live(mix, stacked):
-    from oracle import nets, paddle_shim
-    ref = paddle_shim.import_reference_net("dcn_v2")
-    torch.manual_seed(11)
-    V, D, B, fc = 43, 3, 5, [9, 6]
-    layer = ref.DCN_V2Layer(V, D, 13, 26, fc, 3, stacked, mix, 4, 2)
-    layer.eval()
-    ids = [torch.randint(0, V, (B, 1)) for _ in range(26)]
-    dense = torch.rand(B, 13)
-    named = dict(layer.named_parameters())
-    out = nets.dcn_v2_forward(named, ids, dense, n_fc=len(fc), cross_num=3, is_stacked=stacked,
-                              use_low_rank_mixture=mix, num_experts=2)
-    _same(layer(ids, dense), out, named)
+    from oracle import nets
+    named, i, out, grads = _case("dcn_v2_%d%d" % (mix, stacked))
+    ora = nets.dcn_v2_forward(named, _slots(i["ids"]), i["dense"], n_fc=2, cross_num=3,
+                              is_stacked=stacked, use_low_rank_mixture=mix, num_experts=2)
+    _same(out, grads, ora, named)
 
 
 def test_din_and_wide_deep_live():
-    from oracle import nets, paddle_shim
-    torch.manual_seed(5)
-    ref = paddle_shim.import_reference_net("wide_deep")
-    V, D, B, fc = 37, 6, 4, [8, 4]
-    layer = ref.WideDeepLayer(V, D, 13, 26, fc)
-    ids = [torch.randint(0, V, (B, 1)) for _ in range(26)]
-    dense = torch.rand(B, 13)
-    named = dict(layer.named_parameters())
-    _same(layer(ids, dense), nets.wide_deep_forward(named, ids, dense, len(fc)), named)
+    from oracle import nets
+    named, i, out, grads = _case("wide_deep")
+    _same(out, grads, nets.wide_deep_forward(named, _slots(i["ids"]), i["dense"], 2), named)
 
-    refd = paddle_shim.import_reference_net("din")
-    layer = refd.DINLayer(4, 4, "sigmoid", False, False, 29, 7)
-    B, L = 3, 5
-    hi, hc = torch.randint(0, 29, (B, L)), torch.randint(0, 7, (B, L))
-    ti, tc = torch.randint(0, 29, (B,)), torch.randint(0, 7, (B,))
-    mask = torch.zeros(B, L, 1, dtype=torch.int64)
-    mask[1, 3:] = int(-1e9)
-    named = dict(layer.named_parameters())
-    for i, m in enumerate([m for m in layer.attention_layer if hasattr(m, "weight")]):
-        named["att.linear_%d.weight" % i], named["att.linear_%d.bias" % i] = m.weight, m.bias
-    args = (hi, hc, ti, tc, None, mask, ti.unsqueeze(1).repeat(1, L), tc.unsqueeze(1).repeat(1, L))
-    _same(layer(*args), nets.din_forward(named, *args), named)
-    if os.path.exists("tmp.txt"):
-        os.remove("tmp.txt")
+    named, i, out, grads = _case("din")
+    assert "att.linear_0.weight" in named
+    L = i["hist_item"].shape[1]
+    ti, tc = i["target_item"], i["target_cat"]
+    args = (i["hist_item"], i["hist_cat"], ti, tc, None, i["mask"], ti.unsqueeze(1).repeat(1, L),
+            tc.unsqueeze(1).repeat(1, L))
+    _same(out, grads, nets.din_forward(named, *args), named)
 
 
 @pytest.mark.parametrize("self_interaction,B,d", [(False, 6, 4), (True, 9, 8)])
 def test_dlrm_live(self_interaction, B, d):
     """dlrm/net.py unmodified (train mode: BatchNorm on batch statistics), incl. the
     self_interaction=True branch whose diagonal entries evaluate to 0."""
-    from oracle import nets, paddle_shim
-    ref = paddle_shim.import_reference_net("dlrm")
-    torch.manual_seed(21 + B)
-    V, bot, top = 53, [10, d], [12, 2]
-    layer = ref.DLRMLayer(13, bot, V, d, top, 26, self_interaction=self_interaction)
-    layer.train()
-    ids = [torch.randint(0, V, (B, 1)) for _ in range(26)]
-    dense = torch.rand(B, 13)
-    named = dict(layer.named_parameters())
-    out = nets.dlrm_forward(named, ids, dense, n_bot=len(bot), n_top=len(top),
+    from oracle import nets
+    named, i, out, grads = _case("dlrm_%d" % self_interaction)
+    assert i["ids"].shape == (B, 26) and named["embedding.weight"].shape[1] == d
+    ora = nets.dlrm_forward(named, _slots(i["ids"]), i["dense"], n_bot=2, n_top=2,
                             self_interaction=self_interaction)
-    _same(layer(ids, dense), out, named)
+    _same(out, grads, ora, named)
 
 
-def test_readers_live(tmp_path):
-    """The reference's three Python readers, imported unmodified, against oracle/readers.py and the
-    native parsers on the reference's own bundled sample files."""
-    import importlib.util
-    import sys
-
-    import numpy as np
-
-    from oracle import paddle_shim, readers
+def test_readers_live():
+    """The reference's three Python readers on the reference's own bundled sample files, against
+    oracle/readers.py and the native parsers."""
+    from oracle import readers
     from paddlerec_b200 import dataio
 
-    paddle_shim.install()
-
-    def load(path, name):
-        spec = importlib.util.spec_from_file_location(name, path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        return mod
-
-    sample = os.path.join(REF, "deepfm/data/sample_data/train/sample_train.txt")
-    ds = load(os.path.join(REF, "deepfm/criteo_reader.py"), "ref_criteo_reader").RecDataset([sample], None)
-    ds.inference = False
-    rows = list(ds)
-    ids_ref = np.stack([np.concatenate(r[:27]) for r in rows])
-    dense_ref = np.stack([r[27] for r in rows])
+    gold = np.load(os.path.join(GOLD, "reference_live_readers.npz"))
+    sample = os.path.join(GOLD, "reference_criteo_sample.txt")
+    ids_ref, dense_ref = gold["deepfm/ids"], gold["deepfm/dense"]
     label, ids, dense = dataio.parse_slot_text(open(sample, "rb").read())
     assert np.array_equal(label[:, 0], ids_ref[:, 0]) and np.array_equal(ids, ids_ref[:, 1:])
     assert np.array_equal(dense, dense_ref)
@@ -137,24 +104,14 @@ def test_readers_live(tmp_path):
                                       "dense_feature", 13)
     assert np.array_equal(oi, ids_ref) and np.array_equal(od, dense_ref)
 
-    dcn_sample = os.path.join(REF, "dcn_v2/data/sample_data/sample_train.txt")
-    rows = list(load(os.path.join(REF, "dcn_v2/reader.py"), "ref_dcn_reader").RecDataset([dcn_sample], None))
-    label, ids, dense = dataio.parse_slot_text(open(dcn_sample, "rb").read(), dataio.CRITEO_DCN_V2)
-    assert np.array_equal(ids, np.stack([np.concatenate(r[1:27]) for r in rows]))
+    label, ids, dense = dataio.parse_slot_text(open(sample, "rb").read(), dataio.CRITEO_DCN_V2)
+    assert np.array_equal(ids, gold["dcn_v2/ids"])
     # log(v+1): numpy's and libm's double log may differ in the last place before the float32 cast
-    assert np.allclose(dense, np.stack([r[27] for r in rows]), rtol=2e-7, atol=0)
+    assert np.allclose(dense, gold["dcn_v2/dense"], rtol=2e-7, atol=0)
 
-    din_sample = os.path.join(REF, "din/data/train_data/sample_data.txt")
-    cwd = os.getcwd()
-    os.chdir(tmp_path)                                   # dinReader.py writes ./tmp.txt
-    try:
-        rd = load(os.path.join(REF, "din/dinReader.py"), "ref_din_reader")
-        samples = list(rd.RecDataset([din_sample], {"runner.train_batch_size": 8}))
-    finally:
-        os.chdir(cwd)
+    din_sample = os.path.join(GOLD, "reference_din_sample.txt")
     batches = list(dataio.DinBatchReader([din_sample], 8, as_torch=False))
-    assert len(batches) == len(samples) // 8 > 0
+    assert len(batches) == int(gold["din/n_samples"]) // 8 > 0
     for b, batch in enumerate(batches):
         for j in range(8):
-            want = np.stack([np.asarray(s[j]) for s in samples[8 * b:8 * b + 8]])
-            assert np.array_equal(batch[j], want), (b, j)
+            assert np.array_equal(batch[j], gold["din/b%d/%d" % (b, j)]), (b, j)
