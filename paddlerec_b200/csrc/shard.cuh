@@ -269,10 +269,16 @@ static int launch_shard_fm_grads_push(const float* feat, const float* S, const f
                                       const uint64_t* peer_ptrs_host, int64_t ld_dst, int world,
                                       int64_t B, int F, int Dn, int D, int G, cudaStream_t st);
 
-static int fill_peer_table(PeerTable* t, const uint64_t* peer_ptrs_host, int world) {
+// `align`: bytes of the widest store the kernel issues through the pointers (float4 / float2).
+static int fill_peer_table(PeerTable* t, const uint64_t* peer_ptrs_host, int world, int align) {
   B200_REQUIRE(world >= 1 && world <= kMaxPeers, "shard push: world=%d (max %d)", world, kMaxPeers);
-  for (int r = 0; r < kMaxPeers; ++r)
-    t->base[r] = r < world ? reinterpret_cast<float*>((uintptr_t)peer_ptrs_host[r]) : nullptr;
+  for (int r = 0; r < kMaxPeers; ++r) {
+    const uint64_t p = r < world ? peer_ptrs_host[r] : 0;
+    B200_REQUIRE(r >= world || p != 0, "shard push: receive buffer of rank %d is NULL", r);
+    B200_REQUIRE(p % (uint64_t)align == 0,
+                 "shard push: receive buffer of rank %d is not %d-byte aligned", r, align);
+    t->base[r] = reinterpret_cast<float*>((uintptr_t)p);
+  }
   return B200REC_OK;
 }
 
@@ -280,11 +286,11 @@ static int launch_shard_gather_push(const float* W, int64_t ldw, int D, int64_t 
                                     const int64_t* ids, const int64_t* seg_dev,
                                     const int64_t* dst_dev, const uint64_t* peer_ptrs_host,
                                     int64_t ld_dst, int world, int64_t n, cudaStream_t st) {
-  PeerTable t;
-  int rc = fill_peer_table(&t, peer_ptrs_host, world);
-  if (rc != B200REC_OK) return rc;
   RowShape rs;
   B200_REQUIRE(pick_row_shape(D, &rs), "shard_gather_push: unsupported D=%d", D);
+  PeerTable t;
+  int rc = fill_peer_table(&t, peer_ptrs_host, world, rs.vec * 4);
+  if (rc != B200REC_OK) return rc;
   B200_REQUIRE(ldw >= D && ld_dst >= D && ldw % rs.vec == 0 && ld_dst % rs.vec == 0,
                "shard_gather_push: bad row strides");
   B200_REQUIRE(reinterpret_cast<uintptr_t>(W) % (rs.vec * 4) == 0,
@@ -309,11 +315,11 @@ static int launch_shard_gather_push(const float* W, int64_t ldw, int D, int64_t 
 static int launch_shard_push_rows(const float* rows, int64_t ld, int D, const int64_t* seg_dev,
                                   const int64_t* dst_dev, const uint64_t* peer_ptrs_host,
                                   int64_t ld_dst, int world, int64_t n, cudaStream_t st) {
-  PeerTable t;
-  int rc = fill_peer_table(&t, peer_ptrs_host, world);
-  if (rc != B200REC_OK) return rc;
   RowShape rs;
   B200_REQUIRE(pick_row_shape(D, &rs), "shard_push_rows: unsupported D=%d", D);
+  PeerTable t;
+  int rc = fill_peer_table(&t, peer_ptrs_host, world, rs.vec * 4);
+  if (rc != B200REC_OK) return rc;
   B200_REQUIRE(ld >= D && ld_dst >= D && ld % rs.vec == 0 && ld_dst % rs.vec == 0,
                "shard_push_rows: bad row strides");
   B200_REQUIRE(reinterpret_cast<uintptr_t>(rows) % (rs.vec * 4) == 0,
@@ -341,7 +347,7 @@ static int launch_shard_fm_grads_push(const float* feat, const float* S, const f
                                       const uint64_t* peer_ptrs_host, int64_t ld_dst, int world,
                                       int64_t B, int F, int Dn, int D, int G, cudaStream_t st) {
   PeerTable t;
-  int rc = fill_peer_table(&t, peer_ptrs_host, world);
+  int rc = fill_peer_table(&t, peer_ptrs_host, world, 16);
   if (rc != B200REC_OK) return rc;
   B200_REQUIRE(D > 0 && D % 4 == 0 && G % 4 == 0 && G >= D + 1 && ld_dst >= G && ld_dst % 4 == 0,
                "shard_fm_grads_push: needs D %% 4 == 0 and G %% 4 == 0, G >= D+1 (D=%d G=%d)", D, G);

@@ -482,6 +482,21 @@ def raw_tower_fold_dw(Mx: torch.Tensor, K: int, N: int) -> torch.Tensor:
 
 
 # ---- sharded exchange over NVLink peer memory (csrc/shard.cuh) ----------------------------------
+def _peer_tables(seg_dev: torch.Tensor, dst_dev: torch.Tensor, peer_ptrs, world: int):
+    """The kernels read world+1 entries of seg_dev and world of dst_dev on the device and store
+    through peer_ptrs[0..world): a short table would send rows to addresses read past its end."""
+    seg_dev = _req(seg_dev, torch.int64, "seg_dev")
+    dst_dev = _req(dst_dev, torch.int64, "dst_dev")
+    if seg_dev.numel() != world + 1 or dst_dev.numel() != world:
+        raise _lib.B200RecError(
+            "shard exchange: seg_dev must have world+1 = %d entries and dst_dev world = %d, got %d "
+            "and %d" % (world + 1, world, seg_dev.numel(), dst_dev.numel()))
+    if len(peer_ptrs) < world:
+        raise _lib.B200RecError("shard exchange: %d peer pointers for world=%d"
+                                % (len(peer_ptrs), world))
+    return seg_dev, dst_dev
+
+
 def raw_shard_gather_push(shard: torch.Tensor, recv_ids: torch.Tensor, local_pad: int, D: int,
                           seg_dev: torch.Tensor, dst_dev: torch.Tensor, peer_ptrs, ld_dst: int,
                           world: int) -> None:
@@ -489,6 +504,8 @@ def raw_shard_gather_push(shard: torch.Tensor, recv_ids: torch.Tensor, local_pad
     directly into r's receive buffer (peer_ptrs: ctypes uint64 array of mapped base pointers)."""
     lib = _lib.load()
     shard = _req(shard, torch.float32, "shard") if shard.is_contiguous() else shard
+    recv_ids = _req(recv_ids, torch.int64, "recv_ids")
+    seg_dev, dst_dev = _peer_tables(seg_dev, dst_dev, peer_ptrs, world)
     check(lib.b200rec_shard_gather_push(ptr(shard), shard.stride(0), D, shard.shape[0],
                                         int(local_pad), ptr(recv_ids), ptr(seg_dev), ptr(dst_dev),
                                         peer_ptrs, ld_dst, world, recv_ids.numel(), _stream()),
@@ -506,6 +523,7 @@ def raw_shard_fm_grads_push(feat, S, dfeat_dnn, gy1, gy2, inv_perm, F: int, G: i
     if dfeat_dnn is not None:
         dfeat_dnn = _req(dfeat_dnn, torch.float32, "dfeat_dnn")
     B, N, D = feat.shape
+    seg_dev, dst_dev = _peer_tables(seg_dev, dst_dev, peer_ptrs, world)
     check(lib.b200rec_shard_fm_grads_push(ptr(feat), ptr(S), ptr(dfeat_dnn),
                                           ptr(_req(gy1, torch.float32, "gy1")),
                                           ptr(_req(gy2, torch.float32, "gy2")),
@@ -520,6 +538,7 @@ def raw_shard_push_rows(rows: torch.Tensor, D: int, seg_dev: torch.Tensor, dst_d
     """Requester side of the push: gradient rows in bucket order -> the owners' receive buffers."""
     lib = _lib.load()
     rows = _req(rows, torch.float32, "rows")
+    seg_dev, dst_dev = _peer_tables(seg_dev, dst_dev, peer_ptrs, world)
     check(lib.b200rec_shard_push_rows(ptr(rows), rows.stride(0), D, ptr(seg_dev), ptr(dst_dev),
                                       peer_ptrs, ld_dst, world, rows.shape[0], _stream()),
           "shard_push_rows")

@@ -93,8 +93,9 @@ class PeerBuffers:
 
 
 P2P_MAX_WORLD = 4
-# b200rec_shard_fm_grads_push (K2's sparse half + the push as one kernel): compiled and desk-checked
-# but NOT yet run on a GPU (the round's GPU budget ended first) -> opt-in only.
+# b200rec_shard_fm_grads_push (K2's sparse half + the push as one kernel) stores the same bits as K2 +
+# b200rec_shard_push_rows on one GPU with virtual peers (tests/test_gpu_shard_kernels.py), but the
+# exchange with it has not run across GPUs yet -> opt-in only.
 FUSED_PUSH = os.environ.get("B200REC_FUSED_PUSH", "0") == "1"
 
 

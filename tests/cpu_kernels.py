@@ -52,7 +52,9 @@ def raw_shard_bucketize(ids, world, V):
 def raw_gather(W, ids, pad, D=None):
     W = W if D is None else W[:, :D]
     ok = (ids >= 0) & (ids < W.shape[0]) & (ids != pad)
-    return W[ids.clamp(0, max(W.shape[0] - 1, 0))] * ok.unsqueeze(-1).to(W.dtype)
+    # where, not a multiply by the mask: the kernels store +0.0 for these rows (x * 0 is -0.0 for
+    # a negative x)
+    return torch.where(ok.unsqueeze(-1), W[ids.clamp(0, max(W.shape[0] - 1, 0))], 0.0)
 
 
 def raw_embed_fm_fwd(W, W1, ids, dense, dense_w, dense_w1, pad, want_S=True, D=None):

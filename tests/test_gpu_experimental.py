@@ -1,6 +1,8 @@
-"""Opt-in paths that were written after the round's GPU budget ended and have NOT run on a GPU yet
-(DESIGN.md section 6): ahead-of-time id grouping (B200REC_GROUP_AHEAD) and the fused FM-gradient
-push of the sharded path (B200REC_FUSED_PUSH).  Both must reproduce the default path bit for bit:
+"""Opt-in paths that have NOT run end to end on a GPU yet (DESIGN.md section 6): ahead-of-time id
+grouping (B200REC_GROUP_AHEAD) and the fused FM-gradient push of the sharded path
+(B200REC_FUSED_PUSH; its kernel is tested on one GPU with virtual peers in
+tests/test_gpu_shard_kernels.py, the exchange across GPUs is not).  Both must reproduce the default
+path bit for bit:
 the same kernels compute the same values, only the stream / the number of launches differs.
 
     B200REC_TEST_EXPERIMENTAL=1 python -m pytest tests/test_gpu_experimental.py -m gpu -q

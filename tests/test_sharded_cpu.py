@@ -382,7 +382,8 @@ def _tables_worker(rank, world, port, out_dir):
 def test_peer_memory_exchange_tables(world, tmp_path):
     """The device tables that steer the peer-memory exchange (send_seg / recv_seg / dst_pull /
     dst_push of ShardExchange._bucketize_and_count), replayed with gloo: rows land where K1's `perm`
-    expects them, gradient rows land in the owner's receive segments."""
+    expects them, gradient rows land in the owner's receive segments.  The kernels that consume
+    these tables are tested on one GPU, from the same formulas, in tests/test_gpu_shard_kernels.py."""
     mp.spawn(_tables_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
     assert all(os.path.exists(os.path.join(str(tmp_path), "ok%d" % r)) for r in range(world))
 
@@ -461,8 +462,10 @@ def _peer_worker(rank, world, port, out_dir, bufs, cap, fused_push):
 def test_peer_memory_choreography_on_host_buffers(world, fused_push, tmp_path):
     """The peer-memory pull / push of ShardExchange (and, with fused_push, the one-kernel
     FM-gradient push) replayed on shared host tensors: same oracle, same tolerances as the all-to-all
-    path.  Covers the host logic (tables, buffer offsets, barriers, zero-segment K2 call); the CUDA
-    kernels themselves are covered by tests/test_sharded_gpu.py."""
+    path.  Covers the host logic (tables, buffer offsets, barriers, zero-segment K2 call) with the
+    torch stand-ins of tests/cpu_kernels.py.  The CUDA kernels themselves are compared with those
+    stand-ins and with float64 references on one GPU, with virtual peers, by
+    tests/test_gpu_shard_kernels.py; tests/test_sharded_gpu.py runs them across 2 or more GPUs."""
     B = _batch_for(world)
     cols = (D + 1 + 3) // 4 * 4
     cap = B // world * F + 8
